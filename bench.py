@@ -1,7 +1,7 @@
 """Benchmark of the plane-sweep depth-inference hot path (BASELINE.json metric: fusionnet depth frames/sec at
 256x256 with 64 planes; warp+correlate HBM GB/s vs peak).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--clips B] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--clips B] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one fusionnet keyframe (config c2: 256x256, D=64, 2 measurement frames, recurrent state carried, hidden-
@@ -121,6 +121,23 @@ def measured_peaks():
 
 def log(msg):
     print("[bench] " + msg, file=sys.stderr, flush=True)
+
+
+DUMP_LIMIT_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(out_dir, depth):
+    """Writes the depth maps (clips, H, W) of the timed path's last step, in clip order, as out_dir/depth.npy (float32), so that
+    two builds run with the same arguments can be compared output for output.  When all clips together exceed 64 MB, a fixed
+    seeded sample of whole clips is written instead, still in clip order."""
+    depth = np.ascontiguousarray(depth, dtype=np.float32)
+    keep = max(1, (DUMP_LIMIT_BYTES - 4096) // depth[0].nbytes)      # 4 KiB left for the .npy header
+    if len(depth) > keep:
+        depth = depth[np.sort(np.random.RandomState(0).choice(len(depth), keep, replace=False))]
+    os.makedirs(out_dir, exist_ok=True)
+    path = os.path.join(out_dir, "depth.npy")
+    np.save(path, depth)
+    log("wrote %s %s" % (path, tuple(depth.shape)))
 
 
 class ClockSampler(threading.Thread):
@@ -305,6 +322,8 @@ def run_ours(args, rank, world, local_rank):
     clocks = sampler.summary()
     dev_ms = dev_ms_total
     assert bool(torch.isfinite(pred).all()), "non-finite depth"
+    # the depth maps of the timed path's last step, copied before the other arms reuse the engines' buffers
+    last_depth = pred.detach().float().reshape(B, H, W).clone()
 
     # ---------------- end-to-end arm: pinned host inputs -> modules -> host depth, copies inside the timed region
     frames_host = []
@@ -632,7 +651,9 @@ def run_ours(args, rank, world, local_rank):
     conv_tf = fps / world * CONV_FLOP_PER_KEYFRAME / 1e12          # per GPU
     dtype = "f32" if args.backend == "fp32" else ("f16+f32acc" if args.tc_terms == 1 else "f16x2+f32acc")
     # final depth maps of every clip on every rank (clip order): the trivial gather of independent clips, outside the timed region
-    gathered = sharding.gather_clip_results({c: pred[i] for i, c in enumerate(my_clips)}, B * world, device=dev)
+    gathered = sharding.gather_clip_results({c: last_depth[i] for i, c in enumerate(my_clips)}, B * world, device=dev)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, torch.stack(gathered).cpu().numpy())
     result = {
         "metric": "fusionnet depth frames/sec @256x256x64planes", "value": fps, "unit": "frames/s",
         "n_gpus": world, "steps": args.steps, "warmup": args.warmup, "ms_per_step": dev_ms / args.steps,
@@ -736,29 +757,30 @@ def best_thread_count(oracle, w, clip):
     return best, {str(k): round(v, 3) for k, v in trials.items()}, len(cores)
 
 
-def cpu_baseline(n_frames, weights_which="auto", budget_s=40.0):
-    """The oracle (restatement of the reference's PyTorch-CPU path) on the host cores: a bounded sample of the same workload --
-    up to n_frames recurrent keyframes of ONE c2 clip after one warm-up keyframe, stopping early once budget_s is spent."""
+def cpu_baseline(n_frames, weights_which="auto", budget_s=40.0, warmup=1):
+    """The oracle (restatement of the reference's PyTorch-CPU path) on the host cores: up to n_frames recurrent keyframes of ONE
+    c2 clip after `warmup` untimed keyframes, stopping early once budget_s is spent (budget_s=None: all n_frames).  Returns the
+    record and the depth map (1, H, W) of the last timed keyframe."""
     saved_aff = None
     try:
         saved_aff = os.sched_getaffinity(0)
     except Exception:  # noqa: BLE001
         pass
     saved_threads = torch.get_num_threads()
-    oracle, w, desc, clip = oracle_inputs(n_frames + 1, weights_which)
+    oracle, w, desc, clip = oracle_inputs(warmup + n_frames, weights_which)
     threads, trials, n_phys = best_thread_count(oracle, w, clip)
-    log("cpu baseline: oracle on %d threads, up to %d frames" % (threads, n_frames))
-    times, st = oracle_frames(oracle, w, clip, 0, 1)
+    log("cpu baseline: oracle on %d threads, %d warm-up + up to %d frames" % (threads, warmup, n_frames))
+    _, st = oracle_frames(oracle, w, clip, 0, warmup)      # untimed: they build the recurrent state the timed keyframes start from
     times = []
-    for t in range(1, n_frames + 1):
+    for t in range(warmup, warmup + n_frames):
         dt, st = oracle_frames(oracle, w, clip, t, 1, state=st)
         times += dt
-        if sum(times) > budget_s and len(times) >= 2:
+        if budget_s is not None and sum(times) > budget_s and len(times) >= 2:
             break
     out = {"value": len(times) / sum(times), "unit": "frames/s", "cores": threads, "kind": "port", "frames_run": len(times),
            "thread_trials_s_per_keyframe": trials, "physical_cores": n_phys, "weights": desc,
-           "sample": "%d recurrent keyframes of one c2 clip (256x256, D=64, M=2) after 1 warm-up, torch %s CPU, %d threads pinned to %d physical cores"
-                     % (len(times), torch.__version__, threads, threads)}
+           "sample": "%d recurrent keyframes of one c2 clip (256x256, D=64, M=2) after %d warm-up, torch %s CPU, %d threads pinned to %d physical cores"
+                     % (len(times), warmup, torch.__version__, threads, threads)}
     try:        # SURVEY 8(d): the reference's cost_volume_fusion alone, beside the GPU kernel's roofline entry (never fatal)
         g = torch.Generator().manual_seed(0)
         f1 = torch.randn(1, 32, H // 2, W // 2, generator=g) * 4
@@ -785,7 +807,7 @@ def cpu_baseline(n_frames, weights_which="auto", budget_s=40.0):
         except Exception:  # noqa: BLE001
             pass
     torch.set_num_threads(saved_threads)
-    return out
+    return out, st.previous_depth.reshape(1, H, W).numpy()
 
 
 def gpu_eager_baseline(n_frames=6, weights_which="auto"):
@@ -818,14 +840,16 @@ def gpu_eager_baseline(n_frames=6, weights_which="auto"):
 
 def run_reference(args):
     """The reference's own CPU implementation of the path (oracle port: the reference is pure PyTorch, nothing compiles), all the
-    host threads it can use (best of a small thread sweep), on the GPU arm's workload.  Runs warm-up + steps keyframes for real when
-    that fits ~2 minutes; otherwise as many as fit, and says how many."""
+    host threads it can use (best of a small thread sweep), on the GPU arm's workload and clip: the warm-up keyframes untimed, then
+    exactly `steps` timed keyframes."""
     # torchrun exports OMP_NUM_THREADS=1 to its workers: rank 0 is the only rank doing work here, give it the machine back
     os.environ.pop("OMP_NUM_THREADS", None)
     torch.set_num_threads(max(1, os.cpu_count() or 1))
     t0 = time.perf_counter()
-    base = cpu_baseline(args.warmup + args.steps - 1, args.weights, budget_s=110.0)
+    base, last_depth = cpu_baseline(args.steps, args.weights, budget_s=None, warmup=args.warmup)
     wall = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last_depth)
     fps = base["value"]
     cfg = workload_config(1, base["weights"])
     return {"impl": "reference", "metric": "fusionnet depth frames/sec @256x256x64planes", "value": fps, "unit": "frames/s",
@@ -865,7 +889,12 @@ def main():
                          "while staying at 1.1e-4 over 72 keyframes of the real fixture scene (profiles/r02_drift_*.json, DESIGN.md section 6)")
     ap.add_argument("--pin", type=int, default=1, help="pin each rank's host thread to the CPUs local to its GPU (NVML affinity)")
     ap.add_argument("--gpu-eager", type=int, default=1, help="also time the reference algorithm as PyTorch eager on the GPU (0 to skip)")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the timed steps, write the depth maps of the last timed step of every clip to DIR/depth.npy (float32; "
+                         "a seeded sample of whole clips above 64 MB); --impl reference writes its one clip the same way")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(3, args.warmup)
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -904,7 +933,7 @@ def main():
             except Exception:  # noqa: BLE001
                 pass
             torch.set_num_threads(max(1, os.cpu_count() or 1))
-            result["cpu_baseline"] = cpu_baseline(args.cpu_frames, args.weights)
+            result["cpu_baseline"], _ = cpu_baseline(args.cpu_frames, args.weights)
         print(json.dumps(result))
     if world > 1:
         import torch.distributed as dist

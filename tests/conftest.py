@@ -39,8 +39,8 @@ def cases():
 
 @pytest.fixture(scope="session")
 def golden_ops():
-    import numpy as np
-    return np.load(os.path.join(REPO, "tests", "golden", "ops.npz"))
+    from oracle import npz_parts
+    return npz_parts.load(os.path.join(REPO, "tests", "golden", "ops.npz"))
 
 
 @pytest.fixture(scope="session")

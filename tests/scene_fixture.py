@@ -1,7 +1,6 @@
 """Loader for the committed slice of the reference's fixture scene (tests/golden/scene000, written by
-oracle/make_golden.py) and for the shipped weights (NOT committed: 133 MB; fetched into
-tests/golden/_ref_data/ by tools/fetch_fixtures.py, which __graft_entry__.build() runs in the build
-container; the directory is git-ignored but travels to the GPU box)."""
+oracle/make_golden.py) and for the shipped weights (NOT committed: 133 MB; copied from a checkout of the
+original project into the git-ignored tests/golden/_ref_data/ by tools/fetch_fixtures.py)."""
 import os
 
 import numpy as np
@@ -62,5 +61,6 @@ def load_scene(new_w=320, new_h=256):
                            measurement_poses=[poses[names.index(n)].astype(np.float32) for n in ids[1:]]))
     fx, fy = new_w / float(old[0]), new_h / float(old[1])
     full_K = np.array([[K[0, 0] * fx, 0, K[0, 2] * fx], [0, K[1, 1] * fy, K[1, 2] * fy], [0, 0, 1]], dtype=np.float64)
-    gold = np.load(os.path.join(SCENE, [f for f in os.listdir(SCENE) if f.startswith("golden_predictions")][0]))["predictions"]
+    from oracle import npz_parts
+    gold = npz_parts.load(os.path.join(SCENE, "golden_predictions_first10.npz"))["predictions"]
     return frames, full_K.astype(np.float32), gold

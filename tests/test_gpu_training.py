@@ -24,7 +24,8 @@ def _cuda(x):
 
 @pytest.fixture(scope="module")
 def golden_training():
-    return np.load(os.path.join(REPO, "tests", "golden", "training.npz"))
+    from oracle import npz_parts
+    return npz_parts.load(os.path.join(REPO, "tests", "golden", "training.npz"))
 
 
 # ------------------------------------------------------------------------------------------------ plane sweep

@@ -317,3 +317,19 @@ def test_pixel_pair_formulation_of_the_fp16_sweep_equals_zero_padded_bilinear(or
         for yy, wy in rows:
             got[:, i] += wy * (wl * img[0, :, yy, xa] + wr * img[0, :, yy, xa + 1])
     assert np.abs(got - want).max() <= 1e-5
+
+
+def test_bench_output_dump_is_float32_in_clip_order_and_capped(tmp_path, monkeypatch):
+    import bench
+    depth = np.arange(5 * 4 * 6, dtype=np.float64).reshape(5, 4, 6)
+    bench.dump_outputs(str(tmp_path / "all"), depth)
+    got = np.load(str(tmp_path / "all" / "depth.npy"))
+    assert got.dtype == np.float32 and np.array_equal(got, depth)
+    # above the size limit: the same seeded sample of whole clips every time, in clip order
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", 4096 + 2 * depth[0].size * 4)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), depth)
+    a, b = np.load(str(tmp_path / "a" / "depth.npy")), np.load(str(tmp_path / "b" / "depth.npy"))
+    assert a.shape == (2, 4, 6) and np.array_equal(a, b)
+    rows = [int(r[0, 0]) // depth[0].size for r in a]
+    assert rows == sorted(rows) and all(np.array_equal(r, depth[i]) for r, i in zip(a, rows))

@@ -1,21 +1,23 @@
 """Copies the reference's shipped weight files (parity fixtures, SURVEY.md section 2 row 7) and its test-driver scripts from
-/root/reference into tests/golden/_ref_data/ (git-ignored; travels to the GPU box with the snapshot).
-Run by __graft_entry__.build() in the build container; a no-op where /root/reference is absent."""
+a checkout of the original project into tests/golden/_ref_data/ (git-ignored; 133 MB, too large for the repository).
+
+    python tools/fetch_fixtures.py <deep-video-mvs checkout>      # or DVMVS_REFERENCE_ROOT=<checkout>
+
+The tests that need these files skip without them."""
 import os
 import shutil
 import sys
 
 REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = os.environ.get("DVMVS_REFERENCE_ROOT", "/root/reference")
 
 
-def fetch(verbose=True):
-    if not os.path.isdir(os.path.join(REF, "dvmvs")):
+def fetch(ref, verbose=True):
+    if not os.path.isdir(os.path.join(ref, "dvmvs")):
         if verbose:
-            print("fetch_fixtures: no reference tree at", REF, "- nothing fetched")
+            print("fetch_fixtures: no reference tree at", ref, "- nothing fetched")
         return False
     for net in ("fusionnet", "pairnet"):
-        src = os.path.join(REF, "dvmvs", net, "weights")
+        src = os.path.join(ref, "dvmvs", net, "weights")
         dst = os.path.join(REPO, "tests", "golden", "_ref_data", "weights", net)
         os.makedirs(dst, exist_ok=True)
         for f in sorted(os.listdir(src)):
@@ -25,12 +27,12 @@ def fetch(verbose=True):
                 if verbose:
                     print("fetched", net, f)
     # the reference's test drivers, verbatim, for the "runs unchanged" test (tests/test_gpu_reference_script.py): git-ignored like
-    # the weights, executed from there on the GPU box, never imported by the product
+    # the weights, never imported by the product
     for net in ("fusionnet", "pairnet"):
         dst = os.path.join(REPO, "tests", "golden", "_ref_data", "scripts", net)
         os.makedirs(dst, exist_ok=True)
         for f in ("run-testing.py", "run-testing-online.py"):
-            s = os.path.join(REF, "dvmvs", net, f)
+            s = os.path.join(ref, "dvmvs", net, f)
             if os.path.isfile(s):
                 shutil.copyfile(s, os.path.join(dst, f))
                 if verbose:
@@ -39,4 +41,7 @@ def fetch(verbose=True):
 
 
 if __name__ == "__main__":
-    sys.exit(0 if fetch() else 0)
+    root = sys.argv[1] if len(sys.argv) > 1 else os.environ.get("DVMVS_REFERENCE_ROOT")
+    if not root:
+        sys.exit("usage: python tools/fetch_fixtures.py <deep-video-mvs checkout>")
+    sys.exit(0 if fetch(root) else 1)
